@@ -2,6 +2,7 @@
 """Benchmark of the FACT hot path on B200: autoregressive motion frames/sec (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--mode precise|bf16] [--impl ours|reference]
+                    [--dump-outputs DIR]
 
 A "step" is one autoregressive frame for the whole batch: one full FACT forward (motion encoder, audio encoder,
 12-layer cross-modal stack, head on row 0) over [B,120,225] motion + [B,240,35] audio, plus the shift-by-one
@@ -32,12 +33,22 @@ sys.path.insert(0, ROOT)
 METRIC = "autoregressive motion frames/sec"
 WORKLOAD = "fact_v5_deeper_t10_cm12 autoregressive generate"
 FLOP_PER_FRAME = 80.97e9  # SURVEY.md 8(d): one full forward per generated frame per clip
+DUMP_BYTES = 64 << 20     # cap of --dump-outputs
+
+
+def positive_int(text):
+    v = int(text)
+    if v < 1:
+        raise argparse.ArgumentTypeError(f"must be at least 1, got {v}")
+    return v
 
 
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=12)
+    ap.add_argument("--steps", type=positive_int, default=12,
+                    help="timed steps: AR frames per clip in the generation legs and the batch sweep, optimizer steps "
+                         "in the training leg (the single-clip and CPU legs have their own options)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--batch", type=int, default=128, help="clips per GPU")
     ap.add_argument("--mode", default="precise", choices=["precise", "bf16"])
@@ -59,7 +70,26 @@ def parse():
                     help="frames of the single-clip leg (configs[1]: 1200 = 20 s at 60 fps)")
     ap.add_argument("--kernels-only", action="store_true", help="developer aid: time the hot kernels alone and exit")
     ap.add_argument("--flag", action="append", default=[], help="developer aid: fact_set_flag name=value")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", dest="dump_outputs", metavar="DIR",
+                    help="after the timed steps, write the frame the last timed step generated for each of rank 0's "
+                         "clips to DIR/last_frame.npy (float32, [batch, 225]) for output-for-output comparison of two "
+                         "builds; inputs and weights are seeded, so the same arguments give the same inputs")
+    args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.kernels_only):
+        ap.error("--dump-outputs writes the outputs of the timed generation of --impl ours")
+    return args
+
+
+def dump_outputs(out_dir, name, t):
+    """Save `t` ([rows, ...]) as out_dir/<name>.npy in float32; above DUMP_BYTES a fixed, seeded sample of its rows
+    (sorted row order), so that two runs with the same arguments store the same rows."""
+    import numpy as np
+    a = t.detach().float().cpu().numpy()
+    if a.nbytes > DUMP_BYTES:
+        keep = DUMP_BYTES // (a.nbytes // a.shape[0])
+        a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], keep, replace=False))]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def load_peaks():
@@ -519,7 +549,7 @@ def run_sweep_leg(args, model, dev, world, rank, stream, barrier, max_over_ranks
     precise = model.mode == "precise"
     pts = []
     for B in [int(v) for v in args.sweep.split(",") if v]:
-        k = max(4, min(args.steps, 12 if B <= 128 else 6))
+        k = args.steps
         w = 3
         T = dims.audio.seq_len + w + k - 1
         motion = 0.5 * torch.randn(B, dims.motion.seq_len, dims.motion.feature_dim, device=dev)
@@ -632,6 +662,8 @@ def run_ours(args):
         ms = max_over_ranks(e0.elapsed_time(e1))
         clocks = sampler.stop(t_wall0, t_wall1) if rank == 0 else None
         assert torch.isfinite(hist).all(), "non-finite frames generated"
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, "last_frame", hist[:, -1])
 
         # ---- end-to-end leg: public API, pinned host inputs -> host result, copies inside the timed region
         audio_e2e = audio_h[:, :dims.audio.seq_len + K - 1].contiguous().pin_memory()

@@ -9,7 +9,10 @@ it walks every record and commits
     key: kind, value count, sha256 of the canonical value bytes;
   * tf_written_record.bin : ONE framed record (the smallest, 11 KB: length | crc | payload | crc) exactly as TensorFlow
     wrote it, so that the GPU box (no /root/reference) still reads TensorFlow-written bytes, and the writer can be
-    required to reproduce the frame byte for byte.
+    required to reproduce the frame byte for byte;
+  * tf_written_records.bin : the SAMPLE_RECORDS smallest records of the first file, framed exactly as TensorFlow wrote
+    them and kept in file order (64 KB), so that the tests read a multi-record stream of TensorFlow-written bytes
+    without the source files (the three files hold 2.8 MB of mostly compressed images).
 
     python tests/golden/make_tfrecord_golden.py
 """
@@ -29,6 +32,7 @@ FILES = ["object_detection/test_data/pets_examples.record",
          "object_detection/test_data/snapshot_serengeti_sequence_examples.record",
          "deeplab/testing/pascal_voc_seg/val-00000-of-00001.tfrecord"]
 HERE = os.path.dirname(os.path.abspath(__file__))
+SAMPLE_RECORDS = 4
 
 
 def feature_summary(payload: bytes) -> dict:
@@ -70,6 +74,7 @@ def frames(path):
 def main():
     manifest = {"source_root": BASE, "files": {}}
     smallest = None
+    framed = {}
     for rel in FILES:
         path = BASE + rel
         raw = open(path, "rb").read()
@@ -77,6 +82,7 @@ def main():
         via_reader = list(I.read_tfrecords(path, verify_payload_crc=True))
         for i, (header, lcrc, payload, pcrc) in enumerate(frames(path)):
             assert payload == via_reader[i]
+            framed[rel, i] = header + struct.pack("<I", lcrc) + payload + struct.pack("<I", pcrc)
             recs.append({"length": len(payload), "length_masked_crc32c": lcrc, "payload_masked_crc32c": pcrc,
                          "payload_sha256": hashlib.sha256(payload).hexdigest(), "features": feature_summary(payload)})
             if smallest is None or len(payload) < len(smallest[2]):
@@ -87,9 +93,16 @@ def main():
                            "sha256": hashlib.sha256(smallest[3]).hexdigest()}
     with open(os.path.join(HERE, "tf_written_record.bin"), "wb") as f:
         f.write(smallest[3])
+    first = manifest["files"][FILES[0]]["records"]
+    picked = sorted(sorted(range(len(first)), key=lambda i: first[i]["length"])[:SAMPLE_RECORDS])
+    sample = b"".join(framed[FILES[0], i] for i in picked)
+    manifest["sample"] = {"file": FILES[0], "records": picked, "path": "tf_written_records.bin",
+                          "sha256": hashlib.sha256(sample).hexdigest()}
+    with open(os.path.join(HERE, "tf_written_records.bin"), "wb") as f:
+        f.write(sample)
     with open(os.path.join(HERE, "tfrecord_manifest.json"), "w") as f:
         json.dump(manifest, f, indent=1)
-    print({k: len(v["records"]) for k, v in manifest["files"].items()}, manifest["fixture"])
+    print({k: len(v["records"]) for k, v in manifest["files"].items()}, manifest["fixture"], manifest["sample"])
 
 
 if __name__ == "__main__":
