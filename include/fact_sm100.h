@@ -233,6 +233,18 @@ FACT_API int fact_head_rows(const float* x, long long row_stride, const float* w
 FACT_API int fact_mse(const float* target, const float* pred, float* loss, float* dpred, float* partial, int batch, int t_len,
              int n, int out_dim, float loss_scale, void* stream);
 
+/* Training windows from a device-resident dataset (inputs_util.py:59-107 with the sequences decoded once and motion
+ * already padded to motion_dim): for b < batch, m0 = motion_row[b], a0 = audio_row[b]:
+ *   motion_out[b, t, :] = motion[m0 + t, :]                 t < motion_len
+ *   target_out[b, t, :] = motion[m0 + target_shift + t, :]  t < target_len
+ *   audio_out[b, t, :]  = audio[a0 + t, :]                  t < audio_len
+ * motion is [rows, motion_dim], audio [rows', audio_dim] (64-bit row arithmetic); the caller guarantees every window
+ * lies inside its arena.  batch <= 65535. */
+FACT_API int fact_gather_windows(const float* motion, int motion_dim, const float* audio, int audio_dim,
+                                 const long long* motion_row, const long long* audio_row, int batch, int motion_len,
+                                 int target_shift, int target_len, int audio_len, float* motion_out, float* target_out,
+                                 float* audio_out, void* stream);
+
 /* ---- whole-model entry points --------------------------------------------------------------------------- */
 
 FACT_API size_t fact_workspace_bytes(const fact_dims* dims, int batch, int mode);

@@ -624,3 +624,55 @@ extern "C" int fact_mse(const float* target, const float* pred, float* loss, flo
   }
   return FACT_OK;
 }
+
+// Training windows out of a device-resident dataset (fact_gather_windows).  blockIdx.z picks the output (0 motion
+// input, 1 target, 2 audio input), blockIdx.y the clip; each window is one contiguous span of len * dim floats in both
+// the arena and the output, so the blocks along x copy it with coalesced loads and stores.
+__global__ void __launch_bounds__(256) gather_windows_kernel(
+    const float* __restrict__ motion, int motion_dim, const float* __restrict__ audio, int audio_dim,
+    const long long* __restrict__ motion_row, const long long* __restrict__ audio_row, int motion_len,
+    int target_shift, int target_len, int audio_len, float* __restrict__ motion_out, float* __restrict__ target_out,
+    float* __restrict__ audio_out) {
+  const int b = blockIdx.y;
+  const float* src;
+  float* dst;
+  long long n;
+  if (blockIdx.z == 0) {
+    n = static_cast<long long>(motion_len) * motion_dim;
+    src = motion + motion_row[b] * motion_dim;
+    dst = motion_out + b * n;
+  } else if (blockIdx.z == 1) {
+    n = static_cast<long long>(target_len) * motion_dim;
+    src = motion + (motion_row[b] + target_shift) * motion_dim;
+    dst = target_out + b * n;
+  } else {
+    n = static_cast<long long>(audio_len) * audio_dim;
+    src = audio + audio_row[b] * audio_dim;
+    dst = audio_out + b * n;
+  }
+  const long long stride = static_cast<long long>(gridDim.x) * blockDim.x;
+  for (long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x; i < n; i += stride) dst[i] = src[i];
+}
+
+extern "C" int fact_gather_windows(const float* motion, int motion_dim, const float* audio, int audio_dim,
+                                   const long long* motion_row, const long long* audio_row, int batch, int motion_len,
+                                   int target_shift, int target_len, int audio_len, float* motion_out,
+                                   float* target_out, float* audio_out, void* stream) {
+  FACT_REQUIRE(motion && audio && motion_row && audio_row && motion_out && target_out && audio_out, FACT_ERR_BAD_SHAPE,
+               "fact_gather_windows: null buffer");
+  FACT_REQUIRE(batch > 0 && batch <= 65535 && motion_dim > 0 && audio_dim > 0, FACT_ERR_BAD_SHAPE,
+               "fact_gather_windows: bad shape (batch %d, motion_dim %d, audio_dim %d)", batch, motion_dim, audio_dim);
+  FACT_REQUIRE(motion_len > 0 && target_len > 0 && audio_len > 0 && target_shift >= 0, FACT_ERR_BAD_SHAPE,
+               "fact_gather_windows: bad window (motion_len %d, target_shift %d, target_len %d, audio_len %d)",
+               motion_len, target_shift, target_len, audio_len);
+  long long span = static_cast<long long>(motion_len) * motion_dim;
+  if (static_cast<long long>(audio_len) * audio_dim > span) span = static_cast<long long>(audio_len) * audio_dim;
+  if (static_cast<long long>(target_len) * motion_dim > span) span = static_cast<long long>(target_len) * motion_dim;
+  long long blocks = (span + 1023) / 1024;                       // ~4 floats per thread on the longest window
+  if (blocks > 1024) blocks = 1024;
+  gather_windows_kernel<<<dim3(static_cast<unsigned>(blocks), batch, 3), 256, 0, as_stream(stream)>>>(
+      motion, motion_dim, audio, audio_dim, motion_row, audio_row, motion_len, target_shift, target_len, audio_len,
+      motion_out, target_out, audio_out);
+  FACT_LAUNCH_CHECK("gather_windows_kernel launch");
+  return FACT_OK;
+}

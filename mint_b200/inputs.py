@@ -6,6 +6,8 @@ Reads / writes the TFRecord files produced by the reference's tools/preprocessin
 training: random `start`, motion_input = seq[start:start+120], target = seq[start+120:start+140], audio_input =
 audio[start:start+240]; eval: start = 0 and the FULL audio track.  `create_input` mirrors mint/core/inputs.py:20-123
 (shuffle buffer 100 + repeat + drop_remainder in training; one ordered pass in eval) and yields dicts of NumPy arrays.
+Its training order (training_order) and window starts (window_start) are shared with mint_b200/device_inputs.py, which
+yields the same batches from a dataset decoded once into GPU memory.
 
 TFRecord framing: u64 length | u32 masked-crc32c(length) | payload | u32 masked-crc32c(payload).
 """
@@ -106,6 +108,29 @@ def to_tfexample(motion_sequence, audio_sequence, motion_name: str, audio_name: 
     return ex
 
 
+def float_list_array(float_list) -> np.ndarray:
+    """A FloatList's values as a writable float32 array.  The field is declared packed, so its serialisation is one
+    tag byte, the varint byte count and the little-endian floats -- whatever encoding the record used -- and one
+    np.frombuffer over it replaces np.asarray's element-by-element walk of protobuf's repeated-float container
+    (the bulk of the decoding time of a long sequence)."""
+    raw = float_list.SerializeToString()
+    if not raw:
+        return np.zeros(0, np.float32)
+    if raw[0] != 0x0A:                                          # field 1, length-delimited
+        raise ValueError(f"FloatList serialised with unexpected tag {raw[0]:#x}")
+    n, shift, pos = 0, 0, 1
+    while True:
+        b = raw[pos]
+        pos += 1
+        n |= (b & 0x7F) << shift
+        shift += 7
+        if b < 0x80:
+            break
+    if pos + n != len(raw) or n % 4:
+        raise ValueError(f"FloatList of {len(raw)} bytes has a packed field of {n} bytes at offset {pos}")
+    return np.frombuffer(raw, "<f4", n // 4, pos).astype(np.float32)     # astype copies: writable, own memory
+
+
 def parse_example(record: bytes) -> dict:
     """-> {motion_sequence [T,219], audio_sequence [T',35], motion_name, audio_name} (mint/core/inputs.py:78-94)."""
     ex = Example.FromString(record)
@@ -113,8 +138,7 @@ def parse_example(record: bytes) -> dict:
     out = {}
     for modality in ("motion", "audio"):
         shape = tuple(int(v) for v in f[f"{modality}_sequence_shape"].int64_list.value)
-        out[f"{modality}_sequence"] = np.asarray(f[f"{modality}_sequence"].float_list.value,
-                                                 np.float32).reshape(shape)
+        out[f"{modality}_sequence"] = float_list_array(f[f"{modality}_sequence"].float_list).reshape(shape)
         out[f"{modality}_sequence_shape"] = np.asarray(shape, np.int32)
         out[f"{modality}_name"] = bytes(f[f"{modality}_name"].bytes_list.value[0])
     return out
@@ -185,6 +209,22 @@ def get_modality_to_param_dict(dataset_config) -> dict:
     return out
 
 
+def training_window(modality_to_params: dict) -> int:
+    """Frames a training window spans: motion input, target and audio input all start at the same frame."""
+    mp, ap = modality_to_params["motion"], modality_to_params["audio"]
+    return max(mp["input_length"], mp["target_shift"] + mp["target_length"], ap["input_length"])
+
+
+def window_start(num_frames: int, modality_to_params: dict, rng) -> int:
+    """The random first frame of a training window over a sequence of num_frames frames (inputs_util.py:82-86):
+    one rng.integers(0, T - window + 1) draw."""
+    window = training_window(modality_to_params)
+    hi = num_frames - window + 1
+    if hi <= 0:
+        raise ValueError(f"sequence of {num_frames} frames is shorter than the {window}-frame window")
+    return int(rng.integers(0, hi))
+
+
 def fact_preprocessing(example: dict, modality_to_params: dict, is_training: bool, rng=None) -> dict:
     """mint/utils/inputs_util.py:59-107 on NumPy arrays."""
     ex = dict(example)
@@ -192,12 +232,7 @@ def fact_preprocessing(example: dict, modality_to_params: dict, is_training: boo
     seq = np.pad(ex.pop("motion_sequence"), [[0, 0], [6, 0]])            # 3-dim translation -> 9-dim slot
     audio = ex.pop("audio_sequence")
     if is_training:
-        window = max(mp["input_length"], mp["target_shift"] + mp["target_length"], ap["input_length"])
-        hi = seq.shape[0] - window + 1
-        if hi <= 0:
-            raise ValueError(f"sequence of {seq.shape[0]} frames is shorter than the {window}-frame window")
-        rng = rng or np.random.default_rng()
-        start = int(rng.integers(0, hi))
+        start = window_start(seq.shape[0], modality_to_params, rng or np.random.default_rng())
     else:
         start = 0
     ex["motion_input"] = seq[start:start + mp["input_length"]]
@@ -207,6 +242,33 @@ def fact_preprocessing(example: dict, modality_to_params: dict, is_training: boo
     else:
         ex["audio_input"] = audio
     return ex
+
+
+SHUFFLE_BUFFER = 100        # .shuffle(100) of mint/core/inputs.py
+SHUFFLE_DRAIN = 50          # what is left of the buffer when the last file of an epoch has been read
+
+
+def training_order(num_files: int, file_items, rng):
+    """The order in which training draws items (mint/core/inputs.py: interleave + .shuffle(100) + .repeat()): per epoch
+    a permutation of the files, each file's items in file order through a shuffle buffer of 100 that yields a random
+    item once full, and at the end of an epoch a drain down to 50 items.  file_items(f) gives the items of file f
+    (parsed examples for create_input, sequence indices for create_device_input); the items are opaque here.
+
+    The caller may draw from `rng` between two items (the window start of fact_preprocessing is drawn right after
+    each item leaves the buffer); the generator only calls rng when the next item is asked for, so such draws
+    interleave with its own exactly as they do in create_input.  Ends only if the files hold no items."""
+    buf = []
+    while True:                                                 # .repeat()
+        order = rng.permutation(num_files)                      # interleave(deterministic=False): any file order
+        for fi in order:
+            for item in file_items(fi):
+                buf.append(item)
+                if len(buf) >= SHUFFLE_BUFFER:
+                    yield buf.pop(int(rng.integers(0, len(buf))))
+        if not buf:
+            return
+        while len(buf) > SHUFFLE_DRAIN:
+            yield buf.pop(int(rng.integers(0, len(buf))))
 
 
 def create_input(train_eval_config, dataset_config, num_cpu_threads: int = 2, is_training: bool = True,
@@ -222,18 +284,7 @@ def create_input(train_eval_config, dataset_config, num_cpu_threads: int = 2, is
 
     def examples():
         if is_training:
-            buf = []
-            while True:                                         # .repeat()
-                order = rng.permutation(len(files))             # interleave(deterministic=False): any file order
-                for fi in order:
-                    for rec in read_tfrecords(files[fi]):
-                        buf.append(parse_example(rec))
-                        if len(buf) >= 100:                     # .shuffle(100)
-                            yield buf.pop(int(rng.integers(0, len(buf))))
-                if not buf:
-                    return
-                while len(buf) > 50:
-                    yield buf.pop(int(rng.integers(0, len(buf))))
+            yield from training_order(len(files), lambda fi: map(parse_example, read_tfrecords(files[fi])), rng)
         else:
             for path in files:
                 for rec in read_tfrecords(path):

@@ -21,6 +21,7 @@ SIGNATURES: dict = {
     "fact_train_workspace_bytes": (C.c_size_t, [_vp, _i]),
     "fact_clip_scale": (_i, [_vp, _ll, _vp, _f, _vp]),
     "fact_train_step": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _f, _vp, _vp, C.c_size_t, C.POINTER(_vp), _i, _vp]),
+    "fact_gather_windows": (_i, [_vp, _i, _vp, _i, _vp, _vp, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp]),
 }
 
 

@@ -5,7 +5,8 @@
     python -m torch.distributed.run --nproc-per-node 8 --master-addr 127.0.0.1 trainer.py ...   (sync data parallel)
 
 Data: the TFRecords named by train_dataset.data_files of the config (the reference's own format, read without
-TensorFlow by mint_b200/inputs.py) when that glob matches files; else --data_npz arrays {motion_input, audio_input,
+TensorFlow by mint_b200/inputs.py, decoded once into GPU memory by mint_b200/device_inputs.py) when that glob matches
+files; else --data_npz arrays {motion_input, audio_input,
 target}; else the synthetic generator of SURVEY.md 8d.
 """
 import argparse
@@ -18,7 +19,7 @@ import torch.distributed as dist
 
 import glob
 
-from mint_b200 import config_util, inputs, model_builder, optim
+from mint_b200 import config_util, device_inputs, model_builder, optim
 from mint_b200.trainer import SingleTaskTrainer
 
 
@@ -76,8 +77,9 @@ def main():
     opt = optim.Adam(model, learning_rate=optim.learning_rate_from_config(cfg["train_config"]))
     bs = cfg["train_config"].batch_size                                     # per replica, as in the reference
     if glob.glob(cfg["train_dataset"].data_files):           # trainer.py:140-146: inputs.create_input per replica
+        # the same batches as inputs.create_input(..., seed=rank), decoded once and gathered on the device
         data = ({k: v for k, v in b.items() if k in ("motion_input", "audio_input", "target")}
-                for b in inputs.create_input(cfg["train_config"], cfg["train_dataset"], is_training=True, seed=rank))
+                for b in device_inputs.create_device_input(cfg["train_config"], cfg["train_dataset"], dev, seed=rank))
     elif args.data_npz:
         data = npz_batches(args.data_npz, bs, rank)
     else:
